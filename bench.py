@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- denoising-steps/sec of the BBDM hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg2] [--dump-outputs DIR]
 
 One "step" = one p_sample at the configured batch: UNet forward + fused Brownian-bridge update
 (+ the Gaussian draw), i.e. one iteration of the reference's p_sample_loop
@@ -13,6 +13,10 @@ paired images.  N>1: one process per GPU (torchrun), every rank samples its own 
 Prints ONE JSON line (see the task contract): value (HBM-resident inputs), e2e (host buffers,
 H2D + D2H inside the timed region), roofline (tcgen05 conv kernel family), cpu_baseline
 (oracle port on the host cores, bounded sample), clocks, gpu_launches.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, float32, so that two builds
+can be compared output for output: inputs, weights and noise are seeded, identical from run to run for the same
+arguments.
 """
 from __future__ import annotations
 
@@ -27,7 +31,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 CONFIGS = {
@@ -156,6 +162,23 @@ class ClockSampler:
                 "samples": len(rows), "power_w_max": max(float(r[3]) for r in rows)}
 
 
+DUMP_BYTES = 60 * 10**6          # --dump-outputs in all: under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy in float32.  When they exceed DUMP_BYTES in all, each is replaced by
+    the same share of its elements, at flat indices drawn from a fixed seed (so two runs sample the same places)."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() * 4 for t in arrays.values())
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if total > DUMP_BYTES:
+            k = a.numel() * DUMP_BYTES // total
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:k].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
 def load_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -254,6 +277,7 @@ def run_ends(args, cfg):
     ns.VQGAN = ap.Namespace(params=ap.Namespace(ckpt_path=None, embed_dim=vq["embed_dim"], n_embed=vq["n_embed"],
                                                 ddconfig=ap.Namespace(**vq["ddconfig"]),
                                                 lossconfig=ap.Namespace(target="torch.nn.Identity")))
+    torch.manual_seed(0)          # the constructor's default init (biases) too: identical weights from run to run
     net = LatentBrownianBridgeModel(ns).eval()
     init_weights(net.denoise_fn)
     torch.manual_seed(4321)
@@ -296,6 +320,8 @@ def run_ends(args, cfg):
         e1.record()
         barrier()
         clk = clocks.stop(t0, time.time())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"images": out_host})
     ms = e0.elapsed_time(e1) / args.batches
     if dist is not None:
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
@@ -351,7 +377,11 @@ def main():
     ap.add_argument("--graph", action="store_true", help="also time CUDA-graph replays of the captured sampling step")
     ap.add_argument("--ends", action="store_true", help="latent configs: end-to-end sample() incl. VQGAN encode / decode")
     ap.add_argument("--batches", type=int, default=1, help="--ends: sampled batches in the timed region")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the native implementation only")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         return run_reference_arm(args, cfg)
@@ -359,6 +389,8 @@ def main():
         assert args.config in VQGAN_ENDS, "--ends needs a latent config (cfg3, cfg4, cfg5)"
         return run_ends(args, cfg)
     assert args.warmup >= 3, "timing rules: W >= 3"
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -418,6 +450,7 @@ def main():
             return self._timed_transform("wino_output", super().wino_output, *a, **kw)
 
     BridgeOps.backend_factory = staticmethod(lambda: ProfilingBackend())
+    torch.manual_seed(0)          # the constructor's default init (biases) too: identical weights from run to run
     net = BrownianBridgeModel(namespace(cfg["unet"], cfg["sample_step"])).eval()
     init_weights(net.denoise_fn)
     net = net.to(dev)
@@ -460,10 +493,12 @@ def main():
     t_wall0 = time.time()
     e0.record()
     for i in range(args.steps):
-        x, _ = net.p_sample(x, y, ctx_of(y), (10 + i) % (n_sched - 1))
+        x, x0 = net.p_sample(x, y, ctx_of(y), (10 + i) % (n_sched - 1))
     e1.record()
     barrier()
     t_wall1 = time.time()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"x_prev": x, "x0_recon": x0})        # p_sample's (x_{t-1}, x0 estimate)
     launches = cabi.LAUNCHES["n"] - n0
     ms_dev = max_over_ranks(e0.elapsed_time(e1)) / args.steps
 

@@ -81,6 +81,10 @@ UNET_CONFIGS = {
 }
 
 
+# torch CPU threads the fixtures are generated and checked with (fp32 summation order depends on it)
+GOLDEN_THREADS = 8
+
+
 def bb_namespace(unet: dict, *, num_timesteps=1000, mt_type="linear", objective="grad",
                  loss_type="l1", skip_sample=True, sample_type="linear", sample_step=200,
                  eta=1.0, max_var=1.0):
@@ -156,3 +160,38 @@ def vqgan_state_dict(shapes: dict, seed: int = 4321):
     sd = fill_state_dict(shapes, seed)
     sd["quantize.embedding.weight"] = sd["quantize.embedding.weight"] * 25.0
     return sd
+
+
+# ---- LatentBrownianBridgeModel on the reference's f4 template, shrunk for a CPU test -----------------------------
+def to_namespace(d):
+    """Nested dicts -> nested argparse.Namespace, as the reference's config loader builds ``config.model``."""
+    return argparse.Namespace(**{k: to_namespace(v) if isinstance(v, dict) else v for k, v in d.items()})
+
+
+def lbbdm_small_config(condition_key: str):
+    """``config.model`` of Template-LBBDM-f4.yaml (committed in tests/golden/lbbdm_templates.json) with a 32x32
+    image -> 8x8x3 latent VQGAN, a two-level UNet and a 4-step schedule."""
+    import copy
+    import json
+    import os
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "lbbdm_templates.json")) as f:
+        m = copy.deepcopy(json.load(f)["Template-LBBDM-f4.yaml"]["model"])
+    m["VQGAN"]["params"]["ckpt_path"] = None
+    m["VQGAN"]["params"]["ddconfig"].update(resolution=32, ch=32, ch_mult=(1, 2, 2))
+    m["VQGAN"]["params"]["n_embed"] = 64
+    m["BB"]["params"]["UNetParams"].update(image_size=8, model_channels=32, num_head_channels=32, channel_mult=(1, 2),
+                                           condition_key=condition_key, in_channels=6 if condition_key != "nocond" else 3)
+    m["BB"]["params"]["sample_step"] = 4
+    m["CondStageParams"].update(n_stages=2, in_channels=3, out_channels=3)
+    return to_namespace(m)
+
+
+def lbbdm_state_dict(sd: dict):
+    """Seeded values for every parameter of a LatentBrownianBridgeModel state_dict (UNet, VQGAN, cond stage); the
+    bridge's schedule buffers keep the values given."""
+    out = dict(sd)
+    for prefix, fill in (("denoise_fn.", lambda s: fill_state_dict(s, seed=7)), ("vqgan.", vqgan_state_dict),
+                         ("cond_stage_model.", lambda s: fill_state_dict(s, seed=11))):
+        shapes = {k[len(prefix):]: tuple(v.shape) for k, v in sd.items() if k.startswith(prefix)}
+        out.update({prefix + k: v for k, v in fill(shapes).items()})
+    return out

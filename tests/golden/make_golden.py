@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generate the committed golden fixtures by running the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs an upstream BBDM checkout, named by BBDM_REFERENCE:
 
-    python tests/golden/make_golden.py            # small fixtures (seconds)
-    python tests/golden/make_golden.py --cfg1     # + full-size cfg1 fixture (~1 min CPU)
+    BBDM_REFERENCE=<checkout> python tests/golden/make_golden.py            # small fixtures (seconds)
+    BBDM_REFERENCE=<checkout> python tests/golden/make_golden.py --cfg1     # + full-size cfg1 fixture (~1 min CPU)
 
 Writes ``tests/golden/*.npz`` / ``*.json``.  Weights are never stored: they are
 regenerated from names+shapes by tests/_recipe.fill_state_dict (same code both sides).
@@ -23,7 +23,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 import conftest  # noqa: E402
-from _recipe import UNET_CONFIGS, bb_namespace, fill_state_dict, synth_images  # noqa: E402
+from _recipe import GOLDEN_THREADS, UNET_CONFIGS, bb_namespace, fill_state_dict, synth_images  # noqa: E402
 
 torch.set_grad_enabled(False)
 
@@ -175,14 +175,84 @@ def cfg2_full_size(B=1):
     print("cfg2_b1", f"{os.path.getsize(path) / 1e6:.1f} MB")
 
 
+def reference_contracts():
+    """Everything the CPU tests compare against that needs the reference's own Python modules or config files:
+
+    - the ``model`` section of the three LBBDM templates and the state_dict names / shapes of the reference
+      VQModel built from each (the checkpoint format ``bbdm_b200.vqgan.VQModel`` must load) -> lbbdm_templates.json
+    - the reference's full sampling loop on fresh inputs (tests/test_oracle_pinned.py)
+    - the reference LatentBrownianBridgeModel on the shrunken f4 template with seeded weights
+      (tests/test_latent_model_host.py): state_dict names, parameter count, encode, sample, training loss
+    -> reference_contracts.npz"""
+    import yaml
+    from _recipe import lbbdm_small_config, lbbdm_state_dict
+    conftest.install_reference_shims()
+    from utils import dict2namespace
+    from model.VQGAN.vqgan import VQModel as RefVQ
+    templates = {}
+    for name in ("Template-LBBDM-f4.yaml", "Template-LBBDM-f8.yaml", "Template-LBBDM-f16.yaml"):
+        with open(os.path.join(conftest.REF, "configs", name)) as f:
+            model = yaml.load(f, Loader=yaml.FullLoader)["model"]
+        params = dict(model["VQGAN"]["params"], ckpt_path=None)
+        with torch.device("meta"):
+            vq = RefVQ(**vars(dict2namespace({"p": params}).p))
+        templates[name] = {"model": model, "vqgan_state_dict": {k: list(v.shape) for k, v in vq.state_dict().items()}}
+    with open(os.path.join(HERE, "lbbdm_templates.json"), "w") as f:
+        json.dump(templates, f, indent=1)
+
+    data = {}
+    for unet_name, bkw in (("tiny_pixel", dict(sample_step=20)),
+                           ("tiny_latent", dict(objective="noise", skip_sample=False, num_timesteps=30))):
+        net = build_ref(unet_name, **bkw)
+        shapes = {k: tuple(v.shape) for k, v in net.denoise_fn.state_dict().items()}
+        net.denoise_fn.load_state_dict(fill_state_dict(shapes, seed=99))
+        y = synth_images((2, UNET_CONFIGS[unet_name]["out_channels"], 16, 16), seed=3)
+        torch.manual_seed(7)
+        data[f"{unet_name}_steps"] = net.steps.numpy()
+        data[f"{unet_name}_sample"] = net.sample(y, clip_denoised=False).numpy()
+
+    # a PURE reference pair: load the reference latent module while the dotted base-module name points at the
+    # reference's own BrownianBridgeModel, then restore the overlay
+    name = "model.BrownianBridge.BrownianBridgeModel"
+    overlay = sys.modules.get(name)
+    sys.modules[name] = conftest.load_reference_module("ref_bbdm", "model/BrownianBridge/BrownianBridgeModel.py")
+    try:
+        ref_mod = conftest.load_reference_module("ref_lbbdm", "model/BrownianBridge/LatentBrownianBridgeModel.py")
+    finally:
+        sys.modules.pop(name)
+        if overlay is not None:
+            sys.modules[name] = overlay
+    for ck in ("nocond", "SpatialRescaler"):
+        torch.manual_seed(0)
+        ref = ref_mod.LatentBrownianBridgeModel(lbbdm_small_config(ck)).eval()
+        sd = lbbdm_state_dict(ref.state_dict())
+        ref.load_state_dict(sd)
+        x = synth_images((2, 3, 32, 32), 1)
+        xc = synth_images((2, 3, 32, 32), 2)
+        data[f"{ck}_keys"] = np.array(sorted(sd))
+        data[f"{ck}_n_params"] = np.int64(sum(p.numel() for p in ref.get_parameters()))
+        data[f"{ck}_encode"] = ref.encode(xc, cond=True).numpy()
+        torch.manual_seed(5)
+        data[f"{ck}_sample"] = ref.sample(xc, clip_denoised=False).numpy()
+        torch.manual_seed(9)
+        data[f"{ck}_loss"] = np.float64(ref(x, xc)[0].item())
+    path = os.path.join(HERE, "reference_contracts.npz")
+    np.savez_compressed(path, **data)
+    print("reference_contracts", f"{os.path.getsize(path) / 1e3:.0f} kB")
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--cfg1", action="store_true")
+    ap.add_argument("--contracts-only", action="store_true", help="only the reference model / config contracts")
     ap.add_argument("--cfg2-only", action="store_true", help="only the full-size 256x256 fixture (~2 min CPU)")
     ap.add_argument("--st-only", action="store_true", help="only the SpatialTransformer fixture")
     ap.add_argument("--grads-only", action="store_true", help="only the mid_pixel gradient fixture")
     a = ap.parse_args()
-    torch.set_num_threads(os.cpu_count())
+    torch.set_num_threads(GOLDEN_THREADS)
+    if a.contracts_only:
+        reference_contracts()
+        sys.exit(0)
     if a.cfg2_only:
         cfg2_full_size()
         sys.exit(0)
@@ -199,6 +269,7 @@ if __name__ == "__main__":
     unet_and_psample("mid_pixel", 2, "mid_pixel")
     unet_and_psample("tiny_st", 2, "tiny_st", with_loop=False)          # SpatialTransformer / cross-attention UNet
     mid_pixel_gradients()
+    reference_contracts()
     if a.cfg1:
         unet_and_psample("cfg1", 4, "cfg1", bb_kw=dict(sample_step=100), with_loop=False)
         # BASELINE configs[2..4] UNet shapes at a reduced batch (full channel widths / resolutions)

@@ -78,7 +78,13 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_two_rank_ddp_training_matches_single_process():
+def test_two_rank_ddp_training_matches_single_process(monkeypatch):
+    from bbdm_b200 import optim, train
+    from bbdm_b200.bridge import BridgeOps
+    # the in-process _train() below installs the emulation backend process-wide: undo that when the test ends
+    for cls in (BridgeOps, optim.FusedAdam):
+        monkeypatch.setattr(cls, "backend_factory", cls.__dict__["backend_factory"])
+    monkeypatch.setattr(train, "_BACKEND", train._BACKEND)
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 29000 + os.getpid() % 500

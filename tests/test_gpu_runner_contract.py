@@ -1,9 +1,12 @@
 """-m gpu: the call sequence of the reference runner (runners/BaseRunner.py:59-79,173-192,405-419 and
-runners/DiffusionBasedModelRunners/BBDMRunner.py:21-29,169,240-253) on a real GPU, restated here because the BBDM
-checkout is not present on the GPU box (the unmodified runner itself drives these classes in
-tests/test_dropin_runner.py on the emulation backend): construct -> .to(device) -> apply(weights_init) -> EMA register
+runners/DiffusionBasedModelRunners/BBDMRunner.py:21-29,169,240-253) on a real GPU, restated here because the runner's
+source is not part of this repository; the model and EMA classes are reached through the same imports the runner
+makes (the namespace-package overlays): construct -> .to(device) -> apply(weights_init) -> EMA register
 -> [forward, backward, optimizer step, EMA update] x n -> EMA apply_shadow -> sample -> restore -> image files ->
 checkpoint round trip."""
+import os
+import sys
+
 import numpy as np
 import pytest
 import torch
@@ -13,6 +16,7 @@ from _recipe import UNET_CONFIGS, bb_namespace, synth_images
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
+REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def weights_init(m):                       # what runners/utils.py:35-45 does to Conv2d / Linear modules
@@ -26,6 +30,9 @@ def test_runner_call_sequence_on_gpu(tmp_path):
     from bbdm_b200 import output
     from bbdm_b200.optim import FusedAdam, FusedEMA
     from model.BrownianBridge.BrownianBridgeModel import BrownianBridgeModel
+    from runners.base.EMA import EMA                        # BaseRunner's import: resolves to this repo's overlay
+    assert EMA is FusedEMA and BrownianBridgeModel.__module__ == "model.BrownianBridge.BrownianBridgeModel"
+    assert sys.modules[BrownianBridgeModel.__module__].__file__.startswith(REPO)
     torch.manual_seed(1234)
     ns = bb_namespace(UNET_CONFIGS["mid_pixel"], sample_step=6)
     net = BrownianBridgeModel(ns).to(DEV)
@@ -33,7 +40,7 @@ def test_runner_call_sequence_on_gpu(tmp_path):
     for n, p in net.denoise_fn.named_parameters():          # make the zero-initialised attention projection live
         if n.endswith("proj_out.weight"):
             nn.init.normal_(p.data, 0.0, 0.02)
-    ema = FusedEMA(0.995)
+    ema = EMA(0.995)
     ema.register(net)
     assert list(ema.shadow) == [n for n, p in net.named_parameters() if p.requires_grad]
     opt = FusedAdam(net.get_parameters(), lr=1e-4, weight_decay=0.0, betas=(0.9, 0.999))
@@ -73,7 +80,7 @@ def test_runner_call_sequence_on_gpu(tmp_path):
     ck = torch.load(tmp_path / "ck.pth", map_location="cpu")
     net2 = BrownianBridgeModel(ns).to(DEV)
     net2.load_state_dict(ck["model"])
-    ema2 = FusedEMA(0.995)
+    ema2 = EMA(0.995)
     ema2.register(net2)
     ema2.shadow = ck["ema"]
     ema2.reset_device(net2)

@@ -1,87 +1,58 @@
 """LatentBrownianBridgeModel drop-in (SURVEY section 8 row a23) against the UNMODIFIED reference class:
-same config (Template-LBBDM-f4.yaml shrunk), same weights, random-init frozen VQGAN (the reference's
-own module on both sides) -> encode / forward loss / sample / get_parameters / apply contracts.
-CPU, kernel backend emulated by the oracle (tests only); needs /root/reference."""
+same config (Template-LBBDM-f4.yaml shrunk), same seeded weights -> state_dict names, get_parameters, encode,
+sample, training loss, apply contracts.  The reference's results are stored by tests/golden/make_golden.py in
+reference_contracts.npz.  CPU: the bridge kernels and the VQGAN engine run on the oracle-backed emulation backend
+(tests only)."""
 import os
 
+import numpy as np
 import pytest
 import torch
-import yaml
 
 import conftest
 from _emu_backend import EmuBackend
-from _recipe import fill_state_dict, rel_dev, synth_images
+from _recipe import lbbdm_small_config, lbbdm_state_dict, rel_dev, synth_images
 
-pytestmark = pytest.mark.reference
-
-
-def _config(condition_key):
-    conftest.install_reference_shims()
-    from utils import dict2namespace
-    with open(os.path.join(conftest.REF, "configs", "Template-LBBDM-f4.yaml")) as f:
-        cfg = yaml.load(f, Loader=yaml.FullLoader)
-    m = cfg["model"]
-    m["VQGAN"]["params"]["ckpt_path"] = None
-    dd = m["VQGAN"]["params"]["ddconfig"]
-    dd.update(resolution=32, ch=32, ch_mult=(1, 2, 2))          # f4: 32x32 image -> 8x8x3 latent
-    m["VQGAN"]["params"]["n_embed"] = 64
-    u = m["BB"]["params"]["UNetParams"]
-    u.update(image_size=8, model_channels=32, num_head_channels=32, channel_mult=(1, 2), condition_key=condition_key,
-             in_channels=6 if condition_key != "nocond" else 3)
-    m["BB"]["params"]["sample_step"] = 4
-    m["CondStageParams"].update(n_stages=2, in_channels=3, out_channels=3)
-    return dict2namespace(cfg).model
+GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 @pytest.mark.parametrize("condition_key", ["nocond", "SpatialRescaler"])
 def test_latent_model_matches_reference(condition_key, monkeypatch):
     from bbdm_b200.bridge import BridgeOps
+    from bbdm_b200.cond import SpatialRescaler
+    from bbdm_b200.vqgan_engine import VQGANEngine
     monkeypatch.setattr(BridgeOps, "backend_factory", staticmethod(lambda: EmuBackend()))
-    import sys
-    import model.BrownianBridge.BrownianBridgeModel as overlay_base
+    monkeypatch.setattr(SpatialRescaler, "backend_factory", staticmethod(lambda: EmuBackend()))
     import model.BrownianBridge.LatentBrownianBridgeModel as mine_mod
     assert mine_mod.__file__.startswith(conftest.REPO)
-    # a PURE reference pair: load the reference latent module while the dotted base-module name points at
-    # the reference's own BrownianBridgeModel, then restore the overlay
-    ref_base = conftest.load_reference_module("ref_bbdm", "model/BrownianBridge/BrownianBridgeModel.py")
-    sys.modules["model.BrownianBridge.BrownianBridgeModel"] = ref_base
-    try:
-        ref_mod = conftest.load_reference_module("ref_lbbdm", "model/BrownianBridge/LatentBrownianBridgeModel.py")
-    finally:
-        sys.modules["model.BrownianBridge.BrownianBridgeModel"] = overlay_base
-    assert issubclass(ref_mod.LatentBrownianBridgeModel, ref_base.BrownianBridgeModel)
+    # CPU tensors take the kernel path too, through the emulated backend
+    monkeypatch.setattr(mine_mod.LatentBrownianBridgeModel, "_native", lambda self, fn, x, *a: fn(x, *a))
+    g = {k: v[()] if v.ndim == 0 else v for k, v in
+         np.load(os.path.join(GOLD, "reference_contracts.npz")).items() if k.startswith(condition_key + "_")}
 
     torch.manual_seed(0)
-    mine = mine_mod.LatentBrownianBridgeModel(_config(condition_key)).eval()
-    ref = ref_mod.LatentBrownianBridgeModel(_config(condition_key)).eval()
-    sd = dict(mine.state_dict())
-    shapes = {k: tuple(v.shape) for k, v in mine.denoise_fn.state_dict().items()}
-    for k, v in fill_state_dict(shapes, seed=7).items():
-        sd["denoise_fn." + k] = v
-    assert set(sd) == set(ref.state_dict())                      # identical key set (checkpoint format)
-    ref.load_state_dict(sd)
+    mine = mine_mod.LatentBrownianBridgeModel(lbbdm_small_config(condition_key)).eval()
+    mine.__dict__["_vq_eng"] = VQGANEngine(mine.vqgan, backend=EmuBackend())
+    sd = lbbdm_state_dict(mine.state_dict())
+    assert sorted(sd) == g[f"{condition_key}_keys"].tolist()      # identical key set (checkpoint format)
     mine.load_state_dict(sd)
     assert all(not p.requires_grad for p in mine.vqgan.parameters())
-    n_mine = sum(p.numel() for p in mine.get_parameters())
-    n_ref = sum(p.numel() for p in ref.get_parameters())
-    assert n_mine == n_ref
+    assert sum(p.numel() for p in mine.get_parameters()) == g[f"{condition_key}_n_params"]
 
     x = synth_images((2, 3, 32, 32), 1)
     xc = synth_images((2, 3, 32, 32), 2)
-    assert torch.equal(mine.encode(xc, cond=True), ref.encode(xc, cond=True))
-    torch.manual_seed(5)
-    want = ref.sample(xc, clip_denoised=False)
+    assert rel_dev(mine.encode(xc, cond=True), torch.from_numpy(g[f"{condition_key}_encode"])) < 1e-4
     torch.manual_seed(5)
     got = mine.sample(xc, clip_denoised=False)
+    want = torch.from_numpy(g[f"{condition_key}_sample"])
     assert got.shape == want.shape == (2, 3, 32, 32)
     # the decoder quantises to the nearest codebook entry: an exact match of the decoded image means the
     # latents agreed closely enough to select the same codes everywhere
     assert rel_dev(got, want) < 1e-3
-    torch.manual_seed(9)
-    lw, _ = ref(x, xc)
+    lw = float(g[f"{condition_key}_loss"])
     torch.manual_seed(9)
     lg, log = mine(x, xc)
-    assert abs(float(lw) - float(lg)) < 1e-5 * abs(float(lw))
+    assert abs(lw - float(lg)) < 1e-5 * abs(lw)
     assert lg.requires_grad and "x0_recon" in log
     imgs, one = mine.sample(xc, clip_denoised=False, sample_mid_step=True)
     assert len(imgs) == len(mine.steps) + 1 and len(one) == len(mine.steps) and imgs[0].device.type == "cpu"

@@ -1,12 +1,12 @@
 """Host logic of the sample_to_eval output path (bbdm_b200/output.py) through the emulation backend: byte-identical
 PNG pixels with the reference expression, async writer, opt-in install into the unmodified runner modules."""
 import os
+import sys
 
 import numpy as np
 import pytest
 import torch
 
-import conftest
 from _emu_backend import EmuBackend
 from bbdm_b200 import output as OUT
 
@@ -38,13 +38,18 @@ def test_batch_writer_produces_the_reference_bytes(tmp_path):
     assert np.array_equal(np.asarray(Image.open(tmp_path / "single.png")), _ref_u8(x[3]))
 
 
-@pytest.mark.reference
-def test_install_rebinds_the_runner_functions():
-    conftest.install_reference_shims()
-    import runners.utils as ru
-    old = ru.save_single_image
-    try:
-        assert OUT.install() >= 1
-        assert ru.save_single_image is OUT.save_single_image
-    finally:
-        ru.save_single_image = old
+def test_install_rebinds_the_runner_functions(monkeypatch):
+    """The reference's runners/utils.py defines save_single_image and BBDMRunner.py imports it by name: install()
+    rebinds the name in both modules (stand-ins here, so the test needs no BBDM checkout)."""
+    import types
+
+    def save_single_image(image, save_path, file_name, to_normal=True):
+        raise AssertionError("not rebound")
+
+    for name in ("runners.utils", "runners.DiffusionBasedModelRunners.BBDMRunner"):
+        mod = types.ModuleType(name)
+        mod.save_single_image = save_single_image
+        monkeypatch.setitem(sys.modules, name, mod)
+    assert OUT.install() == 2
+    assert sys.modules["runners.utils"].save_single_image is OUT.save_single_image
+    assert sys.modules["runners.DiffusionBasedModelRunners.BBDMRunner"].save_single_image is OUT.save_single_image

@@ -54,7 +54,10 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_two_rank_sharded_sampling_matches_single_process():
+def test_two_rank_sharded_sampling_matches_single_process(monkeypatch):
+    from bbdm_b200.bridge import BridgeOps
+    # the in-process _build() below installs the emulation backend process-wide: undo that when the test ends
+    monkeypatch.setattr(BridgeOps, "backend_factory", BridgeOps.__dict__["backend_factory"])
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 29500 + os.getpid() % 500
